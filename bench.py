@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — images/sec of IMAGDressing-v1 garment-conditioned sampling (512x512, 50 DDIM steps, CFG) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic inputs: garment-UNet pass + 50 x (CFG-batched
@@ -48,7 +48,34 @@ def parse():
                     help="base = configs[1] (the metric); ipa_controlnet = configs[2]; inpaint = configs[3]")
     ap.add_argument("--height", type=int, default=512)
     ap.add_argument("--width", type=int, default=512)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32), to compare two builds")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times a sample of UNet forwards, not whole steps")
+    return a
+
+
+DUMP_BUDGET_BYTES = 63_000_000  # all files together stay under 64 MB (10^6 bytes) with room for the .npy headers
+
+
+def dump_outputs(d, **arrays):
+    """Write each output as d/<name>.npy in float32. An output past its share of the budget keeps a fixed, seeded sample
+    of its elements (d/<name>.npy, flattened) and their flat indices (d/<name>.index.npy)."""
+    import numpy as np
+
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_BUDGET_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:  # 4-byte value + 8-byte index per kept element
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randperm(a.size, generator=g)[:share // 12].sort().values.numpy()
+            np.save(os.path.join(d, f"{name}.index.npy"), idx)
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(d, f"{name}.npy"), a)
 
 
 def peaks():
@@ -235,9 +262,10 @@ def synth_train_batch(B, dev, rank, pinned, lh, lw):
     return {k: v.to(dev) for k, v in t.items()}
 
 
-def train_record(a, dev, rank, local, world, B, h, w, steps, warm):
+def train_record(a, dev, rank, local, world, B, h, w, steps, warm, dump_dir=None):
     """Training micro-step measured like the sampling workloads: forward + backward of SDModel on the kernels, bucketed NCCL
-    gradient all-reduce overlapped with the backward, AdamW; device events, barrier + synchronize, max over ranks."""
+    gradient all-reduce overlapped with the backward, AdamW; device events, barrier + synchronize, max over ranks.
+    `dump_dir`: write the loss of the last timed step there (dump_outputs)."""
     import torch.distributed as dist
 
     from imagdressing_b200 import _lib, train
@@ -287,9 +315,17 @@ def train_record(a, dev, rank, local, world, B, h, w, steps, warm):
     if rank == 0:
         c.start()
     l0 = _lib.launch_count
-    ms = timed(lambda: step(xd), steps)
+    last = [None]
+
+    def timed_step():
+        last[0] = step(xd)
+
+    ms = timed(timed_step, steps)
     launches = _lib.launch_count - l0
     ck = c.stop() if rank == 0 else None
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, loss=last[0])
+    del last
     ms_e2e = timed(step_e2e, steps)
     _, tf_burst, tf_sus, _ = peaks()
     sps = world * B * steps / (ms * 1e-3)
@@ -607,7 +643,7 @@ def main():
     if a.workload == "train":  # BASELINE.json configs[4]: micro-batch 4 per GPU at 640 x 512 unless overridden
         Bt = a.batch if a.batch != 1 else 4
         h, w = (640, 512) if (a.height, a.width) == (512, 512) else (a.height, a.width)
-        rec = train_record(a, dev, rank, local, world, Bt, h, w, a.steps, max(a.warmup, 5))
+        rec = train_record(a, dev, rank, local, world, Bt, h, w, a.steps, max(a.warmup, 5), a.dump_outputs)
         cb = None
         if rank == 0 and world == 1 and not a.no_cpu_baseline:
             try:
@@ -665,9 +701,17 @@ def main():
     if rank == 0:
         clk.start()
     l0 = _lib.launch_count
-    ms_total = timed(lambda: one_step(x_dev), a.steps)
+    last = [None]
+
+    def timed_step():
+        last[0] = one_step(x_dev)
+
+    ms_total = timed(timed_step, a.steps)
     launches = _lib.launch_count - l0
     clocks = clk.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:  # before any later call can reuse the output buffer
+        dump_outputs(a.dump_outputs, latents=last[0])
+    del last
     one_step_e2e()
     ms_e2e = timed(one_step_e2e, a.steps)
 

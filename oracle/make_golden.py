@@ -1,8 +1,6 @@
-"""Generate tests/golden/processors.safetensors by EXECUTING THE REFERENCE'S OWN CODE (unmodified
-/root/reference/adapter/attention_processor.py and adapter/resampler.py) in fp32 on seeded inputs.
-
-Run in the build container only (the GPU box has no /root/reference):
-    python oracle/make_golden.py
+"""Generate tests/golden/processors/ (safetensors shards, oracle/golden.py) by EXECUTING THE REFERENCE'S OWN CODE
+(unmodified adapter/attention_processor.py and adapter/resampler.py of the reference source tree) in fp32 on seeded inputs:
+    python oracle/make_golden.py <reference source tree>
 The reference file needs two diffusers symbols (attention_processor.py:6-7); oracle/_shim supplies them. The `attn`
 argument is oracle.unet.Attention (the diffusers-0.24 Attention surface the processors touch: to_q/to_k/to_v/
 to_out/heads/spatial_norm/group_norm/norm_cross/residual_connection/rescale_output_factor/prepare_attention_mask).
@@ -14,12 +12,12 @@ import os
 import sys
 
 import torch
-from safetensors.torch import save_file
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle", "_shim"))
-sys.path.insert(0, "/root/reference")
+REF = os.path.abspath(sys.argv[1])
+sys.path.insert(0, REF)
 
 import importlib.util  # noqa: E402
 
@@ -33,12 +31,12 @@ def _load_reference(name, path):
     return mod
 
 
-ref_ap = _load_reference("reference_attention_processor", "/root/reference/adapter/attention_processor.py")  # the reference's file
-ref_rs = _load_reference("reference_resampler", "/root/reference/adapter/resampler.py")
+ref_ap = _load_reference("reference_attention_processor", os.path.join(REF, "adapter", "attention_processor.py"))
+ref_rs = _load_reference("reference_resampler", os.path.join(REF, "adapter", "resampler.py"))
 
 from oracle.unet import Attention  # noqa: E402
 
-assert ref_ap.__file__.startswith("/root/reference"), ref_ap.__file__
+assert ref_ap.__file__.startswith(REF), ref_ap.__file__
 
 G = torch.Generator().manual_seed(1234)
 
@@ -145,7 +143,7 @@ put("refc.proc", rcproc)
 put("refc", out=rcproc(attn2, x, encoder_hidden_states=t, sa_hidden_states={NAME2: g2}),
     out_nosa=rcproc(attn2, x, encoder_hidden_states=t))
 
-dst = os.path.join(ROOT, "tests", "golden", "processors.safetensors")
-save_file(out, dst, metadata={"generator": "oracle/make_golden.py", "reference": "/root/reference @ 2e8a2bd",
-                              "torch": torch.__version__})
-print(f"wrote {dst}: {len(out)} tensors, {os.path.getsize(dst) / 1e6:.2f} MB")
+from oracle import golden  # noqa: E402
+
+n = golden.save_processors(out, metadata={"generator": "oracle/make_golden.py", "torch": torch.__version__})
+print(f"wrote {golden.PROCESSORS}: {len(out)} tensors in {n} shards")

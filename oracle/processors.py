@@ -1,7 +1,7 @@
 """Oracle restatement of the reference's attention processors and Perceiver resampler. TEST INFRASTRUCTURE ONLY.
 
 Each function follows the cited lines of /root/reference/adapter/attention_processor.py and adapter/resampler.py.
-PINNED: tests/test_oracle_golden.py checks these against tests/golden/processors.safetensors, produced by
+PINNED: tests/test_oracle_golden.py checks these against tests/golden/processors/, produced by
 oracle/make_golden.py from the reference's own classes executed (unmodified) in the build container.
 """
 from __future__ import annotations

@@ -203,18 +203,14 @@ def test_sattn_and_refc_drop_ins_match_reference_goldens(monkeypatch):
     """SAttnProcessor2_0 (concat-KV single softmax, reference :103-200) and RefCAttnProcessor2_0 (cross-attention + reference
     branch, :630-744) — installed by no reference script, implemented all the same — through the drop-in classes with the
     kernel wrappers emulated, against goldens produced by the reference's own classes (oracle/make_golden.py)."""
-    import os
-
-    from safetensors import safe_open
-
     import emulated_ops
+    from oracle import golden
 
     emulated_ops.install(monkeypatch)
     import adapter.attention_processor as ap
     from imagdressing_b200.modeling import Attention
 
-    with safe_open(os.path.join(os.path.dirname(__file__), "golden", "processors.safetensors"), "pt") as f:
-        gold = {k: f.get_tensor(k) for k in f.keys()}
+    gold = golden.load_processors()
 
     def load(module, prefix):
         module.load_state_dict({k[len(prefix) + 3:]: v.float() for k, v in gold.items() if k.startswith(prefix + ".w.")})

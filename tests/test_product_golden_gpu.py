@@ -1,24 +1,22 @@
 """GPU: the drop-in adapter/attention_processor.py + adapter/resampler.py (CUDA kernels through the C ABI) against
 the golden vectors produced by the reference's own code. Operands are bf16-exact in the fixture, so the only
 difference is arithmetic: tolerance rel-L2 <= 1e-2 (SURVEY.md §8c)."""
-import os
 
 import pytest
 import torch
-from safetensors import safe_open
 
 from conftest import rel_l2
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), "golden", "processors.safetensors")
 NAME = "down_blocks.0.attentions.0.transformer_blocks.0.attn1.processor"
 TOL = 1e-2
 
 
 @pytest.fixture(scope="module")
 def gold(cuda_device):
-    with safe_open(GOLD, "pt") as f:
-        return {k: f.get_tensor(k).to(cuda_device) for k in f.keys()}
+    from oracle import golden
+
+    return golden.load_processors(cuda_device)
 
 
 def load(module, gold, prefix, dev):
